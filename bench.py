@@ -48,7 +48,12 @@ def parse_args():
                     help="point: one RGB per point shared by the views (default, the BASELINE line); view: per-(view,point) "
                          "colours (V*P0,3) as the reference holds them after shading; shaded: per-point albedo + fused "
                          "shading (one directional light), gradients to albedo, normals and positions")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (image and gradients) as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
 
 
 def load_peaks():
@@ -59,6 +64,24 @@ def load_peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BYTES_PER_ARRAY = 15_000_000     # at most four arrays are written: 60 MB in all
+
+
+def dump_outputs(directory, arrays):
+    """Write each array as float32 <directory>/<name>.npy.  One larger than DUMP_BYTES_PER_ARRAY is stored as a fixed,
+    seeded sample of its rows (leading dimensions flattened, rows kept in order), so that two builds run with the same
+    arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        x = t.detach().float().cpu().numpy()
+        if x.nbytes > DUMP_BYTES_PER_ARRAY:
+            x = x.reshape(-1, x.shape[-1])
+            keep = DUMP_BYTES_PER_ARRAY // (x.itemsize * x.shape[1])
+            x = x[np.sort(np.random.default_rng(0).choice(x.shape[0], keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), x)
 
 
 class ClockSampler:
@@ -377,10 +400,17 @@ def run_ours(a):
         if graphed is not None:
             graphed.replay()
         else:
-            step_resident()
+            last = step_resident()
     e1.record()
     sync_all()
     clocks = sampler.stop()
+    if a.dump_outputs and rank == 0:
+        if graphed is not None:
+            outs = dict(image=graphed.image, grad_points=graphed.grad_points, grad_colours=graphed.grad_colours,
+                        grad_normals=graphed.grad_normals)
+        else:
+            outs = dict(image=last.image, grad_points=pts_d.grad, grad_colours=col_d.grad, grad_normals=nrm_d.grad)
+        dump_outputs(a.dump_outputs, {k: v for k, v in outs.items() if v is not None})
     ms = e0.elapsed_time(e1)
     launches = launches_per_step * a.steps      # kernels executed in the timed region (replayed, not re-launched, under a graph)
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
@@ -474,7 +504,7 @@ def run_ours(a):
         for _ in range(3):
             step_e2e()
         sync_all()
-        n_e2e = max(5, a.steps)
+        n_e2e = a.steps
         f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         f0.record()
         for _ in range(n_e2e):

@@ -4,7 +4,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from dss_b200 import _C
 from dss_b200.ops import SplatParams, render_points
 from tests.util import scene, packed_offsets
-from tests.test_gpu_reference_backward import _reference_fast_backward
+from tests.golden.make_golden_reference import reference_fast_backward as _reference_fast_backward
 from oracle import build_ref
 ref = build_ref.ref_cuda()
 dev = torch.device("cuda:0")

@@ -1,7 +1,7 @@
 """K nearest neighbours within a radius (SURVEY.md section 8(f) row 1).
 
 CPU: the oracle's brute force against golden vectors minted from the reference's own ground truth FRNNBruteForceCPU
-(tests/golden/make_golden_knn.py) and against the compiled witness when present.
+(tests/golden/make_golden_knn.py, tests/golden/make_golden_reference.py).
 GPU: the grid kernel (through the C ABI) against the oracle, bit for bit -- distances AND indices, ties included --
 plus size-independent properties at 1M points."""
 import os
@@ -36,21 +36,18 @@ def test_oracle_knn_reproduces_reference_bruteforce_golden_vectors():
 
 
 def test_oracle_knn_matches_compiled_reference_witness():
-    from oracle import build_ref
-    ref = build_ref.ref_frnn_cpu()
-    if ref is None:
-        pytest.skip("oracle/_ref/dss_ref_frnn_cpu not available")
+    """against what the reference's FRNNBruteForceCPU gave for two ragged clouds (queries and points of different
+    lengths), stored as the valid rows of each cloud back to back"""
+    ref = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference", "knn_bruteforce_ragged.npz"))
     rng = np.random.default_rng(3)
     p1 = rng.uniform(-1, 1, (2, 300, 3)).astype(np.float32)      # queries != points, two clouds of different length
     p2 = rng.uniform(-1, 1, (2, 400, 3)).astype(np.float32)
     l1, l2 = np.array([300, 180], np.int64), np.array([400, 250], np.int64)
-    idxs, dists = ref.frnn_bf_cpu(torch.from_numpy(p1), torch.from_numpy(p2), torch.from_numpy(l1), torch.from_numpy(l2),
-                                  5, 0.4)
     q = np.concatenate([p1[0, :300], p1[1, :180]])
     pts = np.concatenate([p2[0, :400], p2[1, :250]])
     dist, idx = oracle.knn_brute(q, np.array([0, 300]), l1, pts, np.array([0, 400]), l2, 5, 0.4)
-    assert np.array_equal(dist[:300], dists[0, :300].numpy()) and np.array_equal(dist[300:], dists[1, :180].numpy())
-    assert np.array_equal(idx[:300], idxs[0, :300].numpy()) and np.array_equal(idx[300:], idxs[1, :180].numpy())
+    assert np.array_equal(dist, ref["dists"])
+    assert np.array_equal(idx, ref["idxs"])
 
 
 # ------------------------------------------------------------------------------------------------------------
