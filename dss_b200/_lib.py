@@ -49,6 +49,21 @@ class RenderArgs(C.Structure):
     ]
 
 
+DR_LOSS_BLOCKS_PER_VIEW = 128
+DR_LOSS_NUM_SUMS = 5
+
+
+class DrLossArgs(C.Structure):
+    """Mirror of `struct dss_dr_loss_args` (include/dss_b200.h)."""
+    _fields_ = [
+        ("image", vp), ("img", vp), ("mask", vp),
+        ("n_views", C.c_int32), ("image_size", C.c_int32),
+        ("lambda_rgb", C.c_float), ("lambda_silhouette", C.c_float), ("iou_weight", C.c_float),
+        ("reserved0", C.c_int32),
+        ("partials", vp), ("sums", vp), ("terms", vp), ("grad_loss", vp), ("grad_image", vp),
+    ]
+
+
 _SIGNATURES = {
     "dss_version": (C.c_int, []),
     "dss_last_error": (C.c_char_p, []),
@@ -84,6 +99,8 @@ _SIGNATURES = {
     "dss_render_forward": (C.c_int, [vp, C.POINTER(RenderArgs), vp]),
     "dss_render_backward": (C.c_int, [vp, C.POINTER(RenderArgs), vp]),
     "dss_colour_backward": (C.c_int, [vp, C.POINTER(RenderArgs), vp]),
+    "dss_dr_loss_forward": (C.c_int, [vp, C.POINTER(DrLossArgs), vp]),
+    "dss_dr_loss_backward": (C.c_int, [vp, C.POINTER(DrLossArgs), vp]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

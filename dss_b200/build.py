@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libdss_b200.so")
-SOURCES = ["ctx.cu", "binning.cu", "raster_fwd.cu", "backward.cu", "occ_backward.cu", "knn.cu", "render.cu"]
+SOURCES = ["ctx.cu", "binning.cu", "raster_fwd.cu", "backward.cu", "occ_backward.cu", "knn.cu", "render.cu", "loss.cu"]
 HEADERS = ["common.cuh", "kernels.cuh", os.path.join("..", "..", "include", "dss_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

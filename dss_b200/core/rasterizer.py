@@ -23,9 +23,23 @@ from .cloud import clouds_share_points
 from .knn import knn_sq_dists
 
 __all__ = ["PointFragments", "PointsRasterizationSettings", "SurfaceSplatting", "rasterize_elliptical_points",
-           "EllipticalRasterizer", "kMaxPointsPerBin"]
+           "EllipticalRasterizer", "kMaxPointsPerBin", "vrk_h"]
 
 kMaxPointsPerBin = 22   # pytorch3d constant the reference (mis)uses as a bound on bins per side (rasterizer.py:725-730)
+
+
+def vrk_h(points: torch.Tensor, invariant: bool, radius: float = 0.2) -> torch.Tensor:
+    """Variance scale of ONE cloud's splats from its (P,3) points (rasterizer.py:293-402), on the device without a host
+    read-back (the K-NN is csrc/knn.cu), so a CUDA graph can evaluate it on moving points:
+    Vrk_invariant: 0-d clamp(mean_p(0.5 max_{6NN} d^2), 5e-5, 1e-3);  Vrk_isotropic: (P,) clamp(0.5 max_{6NN} d^2, 5e-5, 0.01)."""
+    if points.shape[0] < 7:   # "knn search is unreliable, set sq_dist manually" (rasterizer.py:320-321)
+        h = torch.full((points.shape[0],), 0.5e-3, device=points.device)
+    else:
+        d2 = knn_sq_dists(points.detach(), K=7, radius=radius)[:, 1:]
+        h = 0.5 * d2.max(dim=-1)[0]
+    if invariant:
+        return (h.mean().clamp(5e-5, 1e-3) if h.numel() else h.new_tensor(1e-3)).float()
+    return h.clamp(5e-5, 0.01).float()
 
 
 class PointFragments(NamedTuple):
@@ -127,7 +141,6 @@ class SurfaceSplatting(nn.Module):
         Vrk_isotropic: per point h_p = clamp(0.5 max_{6NN} d^2, 5e-5, 0.01), cached        -> (P,)"""
         rs = kwargs.get("raster_settings", self.raster_settings)
         num = point_clouds.num_points_per_cloud()
-        dev = point_clouds.device
         if not (rs.Vrk_invariant or rs.Vrk_isotropic):
             raise NotImplementedError("anisotropic Vrk (curvature frames + batched SVD, rasterizer.py:256-291) "
                                       "is outside the hot path; use Vrk_invariant or Vrk_isotropic")
@@ -141,15 +154,10 @@ class SurfaceSplatting(nn.Module):
             if shared and n > 0:
                 per_cloud.append(per_cloud[0])
                 continue
-            if pts.shape[0] < 7:   # "knn search is unreliable, set sq_dist manually" (rasterizer.py:320-321)
-                per_cloud.append(torch.full((pts.shape[0],), 0.5e-3, device=dev))
-                continue
-            d2 = knn_sq_dists(pts.detach(), K=7, radius=self.frnn_radius)[:, 1:]
-            per_cloud.append(0.5 * d2.max(dim=-1)[0])
+            per_cloud.append(vrk_h(pts, rs.Vrk_invariant, self.frnn_radius))
         if rs.Vrk_invariant:
-            return torch.stack([h.mean().clamp(5e-5, 1e-3) if h.numel() else h.new_tensor(1e-3)
-                                for h in per_cloud]).float()
-        self._Vrk_h = torch.cat(per_cloud).clamp(5e-5, 0.01).float()
+            return torch.stack(per_cloud)
+        self._Vrk_h = torch.cat(per_cloud)
         return self._Vrk_h
 
     def _get_per_point_info(self, point_clouds, **kwargs):

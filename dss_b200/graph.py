@@ -18,11 +18,15 @@ the records; views whose window does not fit take the direct gather), so a repla
 re-capturing would make it faster again.
 """
 import torch
+import torch.nn.functional as F
 
 from . import _lib
-from .ops import render_points
+from .core.rasterizer import vrk_h
+from .core.texture import camera_centres
+from .ops import Shading, render_points
+from .training.image_loss import _dr_terms
 
-__all__ = ["GraphedRenderStep"]
+__all__ = ["GraphedRenderStep", "GraphedTrainStep"]
 
 
 class GraphedRenderStep:
@@ -91,3 +95,114 @@ class GraphedRenderStep:
         still correct -- overflowing tiles are rasterized from the records -- but a fresh capture will be faster)."""
         now = self._tile_total()
         return self._capacity_at_capture > 0 and now > slack * 1.25 * self._capacity_at_capture
+
+
+class GraphedTrainStep:
+    """One training iteration of a shared cloud seen from N cameras, captured once and replayed:
+    h from the step's own points -> F.normalize(normals) -> render_points -> dr_image_loss -> backward.
+
+        step = GraphedTrainStep(points, normals, colours, proj, view, img, mask, params, h="invariant")
+        for batch in loader:
+            step.load(batch.proj, batch.view, batch.img, batch.mask)   # copy_ into the step's static inputs
+            step.replay()           # step.loss (4,) = {loss, rgb, silhouette, iou}, step.image, step.grad_*
+            optimizer.step()        # over step.parameters(); the step's leaves are updated in place
+
+    The leaves (`step.points`, `step.normals`, `step.colours` -- the albedo with ``shading=``) are fresh copies of what
+    was passed in; give THEM to the optimizer.  Their gradients are `step.grad_points`, `step.grad_normals` (None
+    without shading: the normals then only shape the splats, which the reference does not differentiate) and
+    `step.grad_colours`.  The rendered normals are F.normalize of the raw leaf, as Model._get_normals does
+    (DSS/models/point_modeling.py:84-86), so the normal gradient reaches the raw leaf.
+
+    h: "invariant" or "isotropic" recomputes the splat variance scale from the current points inside the graph, with the
+    rule of SurfaceSplatting._compute_h (Vrk_invariant / Vrk_isotropic, dss_b200.core.rasterizer.vrk_h), as the
+    reference does in every forward; a tensor ((N,) or (N*P0,)) is used as given.
+
+    Frozen at capture, so changing one of them needs a NEW step: the SplatParams (e.g. the radii_backward_scaler schedule
+    of DSS/training/scheduler.py:36-48), the loss weights, the shapes, the light type and shininess.  The optimizer,
+    the projection / repulsion regularisers (their gradient is added to the leaves' before the optimizer step) and
+    any multi-GPU gradient exchange stay outside the graph.
+    """
+
+    def __init__(self, points, normals, colours, proj, view, img, mask, params, h="invariant", shading=None,
+                 lambda_rgb=1.0, lambda_silhouette=1.0, iou_weight=0.01, frnn_radius=0.2, warmup=3, grad_sync=None):
+        dev = _lib.require_cuda(points, normals, colours, proj, view, img, mask)
+        if grad_sync is not None and grad_sync.world_size > 1:
+            raise NotImplementedError("GraphedTrainStep does not capture the multi-GPU gradient exchange; "
+                                      "call render_points(..., grad_sync=...) eagerly")
+        if isinstance(h, str):
+            if h not in ("invariant", "isotropic"):
+                raise ValueError('h must be "invariant", "isotropic" or a tensor, got %r' % h)
+        else:
+            _lib.require_cuda(h)
+            h = h.detach().clone()
+        self.device = dev
+        leaf = lambda t: t.detach().clone().requires_grad_(True)
+        self.points, self.normals, self.colours = leaf(points), leaf(normals), leaf(colours)
+        static = lambda t: t.detach().clone()
+        self.proj, self.view, self.img, self.mask = static(proj), static(view), static(img), static(mask)
+        self._shading = None
+        if shading is not None:
+            self.lights, self.ambient = static(shading.lights), static(shading.ambient)
+            self._shading = (int(shading.light_type), float(shading.shininess))
+        self._h, self._radius, self.params = h, float(frnn_radius), params
+        self._weights = (float(lambda_rgb), float(lambda_silhouette), float(iou_weight))
+        s = torch.cuda.Stream(device=dev)
+        s.wait_stream(torch.cuda.current_stream(dev))
+        with torch.cuda.stream(s):
+            for _ in range(max(1, warmup)):
+                self._eager()
+        torch.cuda.current_stream(dev).wait_stream(s)
+        torch.cuda.synchronize(dev)
+        self._capacity_at_capture = self._tile_total()
+        self._clear_grads()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self.image, self.loss = self._eager()
+        self.grad_points, self.grad_normals, self.grad_colours = self.points.grad, self.normals.grad, self.colours.grad
+
+    def parameters(self):
+        return [self.points, self.normals, self.colours]
+
+    def _clear_grads(self):
+        for t in self.parameters():
+            t.grad = None
+
+    def _splat_h(self):
+        """the variance scale the step renders with, from the current points (see the class docstring)"""
+        N = self.proj.shape[0]
+        if not isinstance(self._h, str):
+            return self._h
+        h0 = vrk_h(self.points, self._h == "invariant", self._radius)
+        return h0.expand(N) if self._h == "invariant" else h0.repeat(N)
+
+    def _eager(self):
+        self._clear_grads()
+        shading = None
+        if self._shading is not None:
+            shading = Shading(self.lights, self.ambient, camera_centres(self.view), *self._shading)
+        out = render_points(self.points, F.normalize(self.normals, dim=-1), self.colours, self.proj, self.view,
+                            self._splat_h(), self.params, shading=shading)
+        terms = _dr_terms(out.image, self.img, self.mask, *self._weights)
+        terms[0].backward()
+        return out.image, terms.detach()
+
+    def load(self, proj, view, img, mask, lights=None, ambient=None):
+        """copy one batch (cameras, targets and, with shading, the light rows) into the step's static inputs"""
+        self.proj.copy_(proj)
+        self.view.copy_(view)
+        self.img.copy_(img)
+        self.mask.copy_(mask)
+        if lights is not None or ambient is not None:
+            if self._shading is None:
+                raise RuntimeError("this step was captured without shading")
+            if lights is not None:
+                self.lights.copy_(lights)
+            if ambient is not None:
+                self.ambient.copy_(ambient)
+
+    def replay(self):
+        self.graph.replay()
+        return self.loss
+
+    _tile_total = GraphedRenderStep._tile_total
+    stale = GraphedRenderStep.stale

@@ -16,7 +16,7 @@ from typing import NamedTuple, Optional
 import torch
 import torch.nn as nn
 
-__all__ = ["BaseLoss", "L1Loss", "L2Loss", "SurfaceLoss", "ProjectionLoss", "RepulsionLoss", "KNN"]
+__all__ = ["BaseLoss", "L1Loss", "L2Loss", "IouLoss", "SurfaceLoss", "ProjectionLoss", "RepulsionLoss", "KNN"]
 
 
 class KNN(NamedTuple):
@@ -90,6 +90,18 @@ class L2Loss(BaseLoss):
         if weights is not None:
             loss = loss * weights
         return loss[mask] if mask is not None else loss
+
+
+class IouLoss(BaseLoss):
+    """losses.py:498-514: 1 - intersection / union per batch element (dims 1.. summed); the reduction then runs over
+    the batch.  The trainer builds it with ``reduction="mean", channel_dim=None`` (trainer.py:138) and calls it as
+    ``iou_loss(mask_gt, mask_pred)``; dss_b200.training.image_loss fuses that call into a CUDA op."""
+
+    def compute(self, predict, target, **kwargs):
+        dims = tuple(range(predict.ndimension())[1:])
+        intersect = (predict * target).sum(dims)
+        union = (predict + target - predict * target).sum(dims)
+        return 1.0 - intersect / eps_denom(union)
 
 
 def _padded_to_packed(x, lengths):

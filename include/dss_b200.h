@@ -293,6 +293,43 @@ DSS_API int dss_colour_backward(dss_ctx *ctx, const dss_render_args *args, void 
 /* per-(point,view) preprocess only (rasterizer.py:443-565 fused): writes ndc, ellipse, radii, scaler. */
 DSS_API int dss_preprocess(dss_ctx *ctx, const dss_render_args *args, void *stream);
 
+/* ---- image objective of a training step (SURVEY.md section 8(f) row 5) ------------------------------
+ * Trainer.calc_dr_loss (DSS/training/trainer.py:332-376) with its L1Loss and IouLoss (DSS/training/losses.py:130-137,
+ * 498-514), fused and without a host read-back.  With m the GT mask, alpha the rendered occupancy, d = pred - GT per
+ * rgb channel and sel = (m != 0) & (alpha != 0):
+ *   M      = number of sel pixels over all views
+ *   L_rgb  = (1/M) sum_sel sum_c |d_c|, 0 when M == 0
+ *   L_mask = mean |m - alpha| over all N*S*S pixels
+ *   L_iou  = mean_n (1 - I_n / eps_denom(U_n)),  I_n = sum m alpha,  U_n = sum (m + alpha - m alpha)  (pixels of view n)
+ *   L_sil  = iou_weight * L_iou + L_mask
+ *   L      = lambda_rgb * L_rgb + lambda_silhouette * L_sil
+ * The forward writes terms = {L, L_rgb, L_sil, L_iou} and the per-view sums the backward needs; the backward writes
+ * d L / d image as torch autograd gives it for the reference expression (|x|' = 0 at 0, no gradient through U_n where
+ * eps_denom clamps it).  Block partials are combined in a fixed order in fp64: bit-reproducible, no atomics, no
+ * allocation, no synchronisation (capturable in a CUDA graph). */
+#define DSS_DR_LOSS_BLOCKS_PER_VIEW 128
+#define DSS_DR_LOSS_NUM_SUMS 5
+typedef struct dss_dr_loss_args {
+    const float *image;            /* (N,S,S,4) rendered rgb + occupancy alpha, 16-byte aligned                 */
+    const float *img;              /* (N,3,S,S) GT colour planes (the data batch's layout: no permute needed)   */
+    const float *mask;             /* (N,S,S) GT mask (an (N,1,S,S) tensor has the same layout)                 */
+    int32_t n_views;               /* N                                                                         */
+    int32_t image_size;            /* S                                                                         */
+    float lambda_rgb;
+    float lambda_silhouette;
+    float iou_weight;              /* 0.01 in the reference (trainer.py:368)                                    */
+    int32_t reserved0;
+    double *partials;              /* scratch, N * DSS_DR_LOSS_BLOCKS_PER_VIEW * DSS_DR_LOSS_NUM_SUMS doubles      */
+    double *sums;                  /* (N+1, DSS_DR_LOSS_NUM_SUMS): row n {M_n, sum |d|, sum |m - alpha|, I_n, U_n} of
+                                      view n, row N the totals; written by the forward, read by the backward      */
+    float *terms;                  /* (4,) forward output {L, L_rgb, L_sil, L_iou}                               */
+    const float *grad_loss;        /* backward: d (objective) / d L, one float in device memory                 */
+    float *grad_image;             /* backward output (N,S,S,4), fully written, 16-byte aligned                 */
+} dss_dr_loss_args;
+
+DSS_API int dss_dr_loss_forward(dss_ctx *ctx, const dss_dr_loss_args *args, void *stream);
+DSS_API int dss_dr_loss_backward(dss_ctx *ctx, const dss_dr_loss_args *args, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
